@@ -2,6 +2,7 @@
 """Benchmark: env-steps/s of the batched Melting Pot hot path on B200 (BASELINE.json metric).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--config 2|3|4|5] [--gather-obs]
+                  [--dump-outputs DIR]
 
 A "step" is one pass of the hot path (state transition + all observations rendered) over one batch of env
 instances per GPU under uniform-random actions. --config picks the BASELINE.json configuration:
@@ -354,6 +355,42 @@ def time_job(job, K, Wm, dist, sampler=None):
   return ev0.elapsed_time(ev1), job.eng.launch_count() - launches0
 
 
+DUMP_ENVS = 16            # env instances per run whose images --dump-outputs writes (a whole batch's run to gigabytes)
+DUMP_LIMIT = 64 << 20     # bytes --dump-outputs may write in one run, over all ranks and substrates
+
+
+def dump_outputs(job, out_dir, prefix, n_envs, budget):
+  """Writes what the last timed step handed its caller as `out_dir/<prefix><name>.npy` (float32 images, float64 else):
+  reward, discount, step_type, scalar_obs and event_count of every env, and rgb, world_rgb and events (unused slots
+  zeroed) of a fixed, seeded sample of `n_envs` envs, whose indices are `sample_envs`. Writes nothing and exits if
+  that is more than `budget` bytes; returns the bytes written."""
+  import numpy as np
+  import torch
+  eng = job.eng
+  idx = np.sort(np.random.default_rng(0).choice(job.B, size=min(n_envs, job.B), replace=False))
+  sel = torch.as_tensor(idx, device=job.dev)
+  events = eng.events[sel].cpu().numpy()
+  used = np.arange(events.shape[1])[None, :] < eng.event_count[sel].cpu().numpy()[:, None]
+  arrays = {
+      'reward': eng.reward.cpu().numpy(), 'discount': eng.discount.cpu().numpy(),
+      'step_type': eng.step_type.cpu().numpy().astype(np.float64),
+      'scalar_obs': eng.scalar_obs[:eng.num_scalar_obs].cpu().numpy(),
+      'event_count': eng.event_count.cpu().numpy().astype(np.float64),
+      'sample_envs': idx.astype(np.float64),
+      'rgb': eng.rgb[sel].cpu().numpy().astype(np.float32),
+      'world_rgb': eng.world_rgb[sel].cpu().numpy().astype(np.float32),
+      'events': np.where(used[..., None], events, 0).astype(np.float64),
+  }
+  total = sum(a.nbytes for a in arrays.values())
+  if total > budget:
+    raise SystemExit(f'bench.py: --dump-outputs would write {total} bytes for {prefix[:-1]}, over the {budget} left of the '
+                     f'{DUMP_LIMIT} bytes a run may write')
+  os.makedirs(out_dir, exist_ok=True)
+  for name, a in arrays.items():
+    np.save(os.path.join(out_dir, f'{prefix}{name}.npy'), a)
+  return total
+
+
 def render_roofline(job, K, Wm):
   """The render kernel alone: CUDA events around each launch on the launching stream."""
   import torch
@@ -489,6 +526,7 @@ def run_b200(args, rank, world, local_rank):
 
   sampler = ClockSampler(gpu_selector(local_rank)) if rank == 0 else None
   per_job, elapsed_ms, launches, env_steps = [], 0.0, 0, 0
+  dumped = 0
   shard = None
   e2e = e2e_scalars = gather = None
   first_job = None
@@ -497,6 +535,10 @@ def run_b200(args, rank, world, local_rank):
     ms, n_l = time_job(job, K, Wm, dist if single else None, sampler if ji == 0 else None)
     if ji == 0 and sampler is not None:
       clocks = sampler.stop()
+    if args.dump_outputs:  # before anything below steps the engine again; each rank keeps to its share of the limit
+      prefix = (f'rank{rank}.' if world > 1 else '') + f'{name}.'
+      dumped += dump_outputs(job, args.dump_outputs, prefix, max(1, DUMP_ENVS // (world * len(my_jobs))),
+                             DUMP_LIMIT // world - dumped)
     elapsed_ms += ms
     launches += n_l
     env_steps += B * K
@@ -616,7 +658,12 @@ def main():
   ap.add_argument('--ref-seconds', type=float, default=15.0, help='CPU arm / cpu_baseline: seconds of oracle work to time')
   ap.add_argument('--no-cpu-baseline', action='store_true')
   ap.add_argument('--gather-obs', action='store_true', help='also measure steps with the stacked-observation gather over NVLink')
+  ap.add_argument('--dump-outputs', metavar='DIR', help='write what the last timed step computed to DIR/<substrate>.<name>.npy, '
+                                                        'at most 64 MB per run (seeded inputs: two builds can be compared '
+                                                        'output for output; --impl b200 only)')
   args = ap.parse_args()
+  if args.dump_outputs and args.impl != 'b200':
+    ap.error('--dump-outputs writes the outputs of the b200 path; --impl reference computes none to compare')
   rank = int(os.environ.get('RANK', '0'))
   world = int(os.environ.get('WORLD_SIZE', '1'))
   local_rank = int(os.environ.get('LOCAL_RANK', '0'))

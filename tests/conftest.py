@@ -8,11 +8,6 @@ if ROOT not in sys.path:
   sys.path.insert(0, ROOT)
 
 
-# Tests that compile from / compare with the reference name the checkout explicitly (the product never guesses one).
-if os.path.isdir('/root/reference/meltingpot/configs'):
-  os.environ.setdefault('MELTINGPOT_REFERENCE_ROOT', '/root/reference')
-
-
 def pytest_configure(config):
   config.addinivalue_line('markers', 'gpu: needs a real B200 (run with -m gpu)')
 

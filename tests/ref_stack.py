@@ -95,26 +95,32 @@ def actions_for(name, players, num_actions, steps=STEPS):
   return rng.integers(0, num_actions, size=(steps, players))
 
 
+def _build_reference_env(name, players, seed):
+  """Inside reference_stack_on_oracle(): the reference's meltingpot.substrate.build(name) with default roles and the env
+  seed pinned to `seed`. Returns (config, env)."""
+  import importlib
+  ref_substrate = importlib.import_module('meltingpot.substrate')
+  ref_builder = importlib.import_module('meltingpot.utils.substrates.builder')
+  config = ref_substrate.get_config(name)
+  roles = (tuple(config.default_player_roles)[0],) * players
+  original = ref_builder.builder
+  ref_builder.builder = lambda settings, **kw: original(settings, env_seed=seed, **kw)  # pin the seed builder.py would draw
+  state = random.getstate()
+  try:
+    build_seed = substrates.BUILD_SEEDS.get(name)
+    if build_seed is not None:
+      random.seed(build_seed)  # configs that draw their map from Python's `random` (coins.py:45-84)
+    return config, ref_substrate.build(name, roles=roles)
+  finally:
+    random.setstate(state)
+    ref_builder.builder = original
+
+
 def run_reference_stack(name, players, steps=STEPS, seed=SEED):
   """Builds `name` through the reference's meltingpot.substrate.build (its configs, builder.py, wrappers, Substrate) on
   the oracle-backed dmlab2d module and returns the fixture record."""
   with reference_stack_on_oracle():
-    import importlib
-    ref_substrate = importlib.import_module('meltingpot.substrate')
-    ref_builder = importlib.import_module('meltingpot.utils.substrates.builder')
-    config = ref_substrate.get_config(name)
-    roles = (tuple(config.default_player_roles)[0],) * players
-    original = ref_builder.builder
-    ref_builder.builder = lambda settings, **kw: original(settings, env_seed=seed, **kw)  # pin the seed builder.py would draw
-    state = random.getstate()
-    try:
-      build_seed = substrates.BUILD_SEEDS.get(name)
-      if build_seed is not None:
-        random.seed(build_seed)  # configs that draw their map from Python's `random` (coins.py:45-84)
-      env = ref_substrate.build(name, roles=roles)
-    finally:
-      random.setstate(state)
-      ref_builder.builder = original
+    config, env = _build_reference_env(name, players, seed)
     try:
       rec = {'substrate': name, 'players': players, 'seed': seed, 'class': type(env).__module__ + '.' + type(env).__name__,
              'action_table': [dict(a) for a in compiler._plain(config.action_set)],  # pylint: disable=protected-access
@@ -136,3 +142,49 @@ def run_reference_stack(name, players, steps=STEPS, seed=SEED):
     finally:
       env.close()
   return rec
+
+
+def describe_raw_timestep(ts):
+  """What a fixture keeps of one dmlab2d-level TimeStep (flat "{i}.RGB", "{i}.REWARD", ..., "WORLD.RGB" observation)."""
+  return {'step_type': int(ts.step_type), 'reward': None if ts.reward is None else float(ts.reward),
+          'discount': None if ts.discount is None else float(ts.discount),
+          'observation': {k: _sha(v) if np.asarray(v).ndim else float(v) for k, v in sorted(ts.observation.items())}}
+
+
+def record_dmlab2d_stream(name, players, steps=12, seed=SEED):
+  """The raw stream the reference's innermost ObservablesWrapper emits (observables_wrapper.py:43-58) on
+  observables().dmlab2d while its stack plays `actions_for(...)`: the action dicts its discrete-action and multiplayer
+  wrappers hand to dmlab2d, and the flat TimeSteps dmlab2d returns."""
+  with reference_stack_on_oracle():
+    _, env = _build_reference_env(name, players, seed)
+    raw_ts, raw_act = [], []
+    env.observables().dmlab2d.timestep.subscribe(raw_ts.append)
+    env.observables().dmlab2d.action.subscribe(raw_act.append)
+    try:
+      acts = actions_for(name, players, env.action_spec()[0].num_values, steps)
+      env.reset()
+      for t in range(steps):
+        env.step([int(a) for a in acts[t]])
+    finally:
+      env.close()
+  assert len(raw_ts) == steps + 1 and len(raw_act) == steps
+  return {'substrate': name, 'players': players, 'seed': seed, 'actions': acts.tolist(),
+          'raw_actions': [{k: int(v) for k, v in sorted(a.items())} for a in raw_act],
+          'raw_timesteps': [describe_raw_timestep(ts) for ts in raw_ts]}
+
+
+def check_raw_timestep(ts, rec, players, env=None):
+  """A dmlab2d-level TimeStep (from lab2d_env.Environment) against one step of a ref_stack_<name>.json fixture; with
+  `env`, its events() too."""
+  assert int(ts.step_type) == rec['step_type']
+  assert (0.0 if ts.discount is None else ts.discount) == rec['discount']
+  for i in range(players):
+    assert float(ts.observation[f'{i + 1}.REWARD']) == rec['reward'][i]
+    for key, value in rec['players'][i].items():
+      if key == 'COLLECTIVE_REWARD':  # added by the reference's wrapper stack, not the dmlab2d module
+        continue
+      obs = ts.observation['WORLD.RGB' if key == 'WORLD.RGB' else f'{i + 1}.{key}']
+      assert (_sha(obs) if np.asarray(obs).ndim else float(obs)) == value, (key, i)
+  if env is not None:
+    events = sorted([n, [float(x) if isinstance(x, np.ndarray) else x.decode() for x in p]] for n, p in env.events())
+    assert events == rec['events']

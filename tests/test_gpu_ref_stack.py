@@ -61,17 +61,30 @@ def test_engine_backed_dmlab2d_module_from_flattened_settings(name):
   P = want['players']
   with lab2d_env.Environment(env=lab, observation_names=lab.observation_names(), seed=lab.env_seed) as env:
     assert isinstance(env._backend, lab2d_env.EngineBackend)  # the CUDA engine, not a stand-in
-    def check(ts, rec):
-      assert int(ts.step_type) == rec['step_type']
-      assert (0.0 if ts.discount is None else ts.discount) == rec['discount']
-      for i in range(P):
-        assert float(ts.observation[f'{i + 1}.REWARD']) == rec['reward'][i]
-        for key, value in rec['players'][i].items():
-          if key == 'COLLECTIVE_REWARD':
-            continue
-          obs = ts.observation['WORLD.RGB' if key == 'WORLD.RGB' else f'{i + 1}.{key}']
-          assert (ref_stack._sha(obs) if np.asarray(obs).ndim else float(obs)) == value, (key, i)
-    check(env.reset(), want['steps'][0])
+    ref_stack.check_raw_timestep(env.reset(), want['steps'][0], P)
     for t, acts in enumerate(want['actions']):
       action = {f'{i + 1}.{k}': np.int32(v) for i, a in enumerate(acts) for k, v in want['action_table'][a].items()}
-      check(env.step(action), want['steps'][t + 1])
+      ref_stack.check_raw_timestep(env.step(action), want['steps'][t + 1], P)
+
+
+def test_substrate_dmlab2d_observables_equal_the_reference_stacks_stream():
+  # observables().dmlab2d (built by flat_action / flat_timestep) against the raw stream the reference's own stack
+  # emitted there for the same actions (tests/golden/dmlab2d_stream_clean_up.json, tools/make_ref_stack_golden.py).
+  from meltingpot import substrate
+  with open(os.path.join(ROOT, 'tests', 'golden', 'dmlab2d_stream_clean_up.json')) as f:
+    want = json.load(f)
+  raw_ts, raw_act = [], []
+  with substrate.build(want['substrate'], roles=('default',) * want['players'], env_seed=want['seed']) as env:
+    env.observables().dmlab2d.timestep.subscribe(raw_ts.append)
+    env.observables().dmlab2d.action.subscribe(raw_act.append)
+    env.reset()
+    for acts in want['actions']:
+      env.step(acts)
+  assert [{k: int(v) for k, v in a.items()} for a in raw_act] == want['raw_actions']
+  assert len(raw_ts) == len(want['raw_timesteps'])
+  for t, (ts, rec) in enumerate(zip(raw_ts, want['raw_timesteps'])):
+    got = ref_stack.describe_raw_timestep(ts)
+    assert (got['step_type'], got['reward'], got['discount']) == (rec['step_type'], rec['reward'], rec['discount']), t
+    assert set(got['observation']) <= set(rec['observation']), t  # (the raw env offers every observation; the wrappers select)
+    for key, value in got['observation'].items():
+      assert value == rec['observation'][key], (t, key)

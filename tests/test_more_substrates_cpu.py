@@ -14,6 +14,7 @@ from meltingpot_b200 import blob as mpb
 from meltingpot_b200 import compiler
 from meltingpot_b200 import substrate
 from meltingpot_b200 import substrates
+from tests import reference_configs
 
 
 CASES = [('territory__open', 9), ('territory__inside_out', 5), ('commons_harvest__closed', 7), ('commons_harvest__partnership', 7), ('coins', 2), ('coop_mining', 6)]
@@ -32,22 +33,20 @@ def test_registered_with_default_roles(name, players):
   assert 'default' in set(cfg.valid_roles)
 
 
-@pytest.mark.skipif(compiler.reference_root() is None, reason='needs the reference checkout')
 @pytest.mark.parametrize('name,players', CASES)
 def test_committed_blob_is_what_the_compiler_emits(name, players):
-  fresh = compiler.compile_substrate(name, ('default',) * players, build_seed=substrates.BUILD_SEEDS.get(name))
+  # compiled from the settings the reference's config builds (recorded under tests/golden)
+  fresh = reference_configs.compile_recorded(name, build_seed=substrates.BUILD_SEEDS.get(name))
   assert fresh == substrates.load_blob(name, ('default',) * players)
 
 
-@pytest.mark.skipif(compiler.reference_root() is None, reason='needs the reference checkout')
 @pytest.mark.parametrize('name,players', CASES)
 def test_specs_follow_the_reference_config(name, players):
-  ref = compiler.load_reference_config(name)
+  ref = reference_configs.config(name)
   cfg = substrate.get_config(name)
-  want = ref.timestep_spec.observation['WORLD.RGB'].shape
-  assert tuple(cfg.timestep_spec.observation['WORLD.RGB'].shape) == tuple(want)
-  assert tuple(cfg.timestep_spec.observation['RGB'].shape) == tuple(ref.timestep_spec.observation['RGB'].shape)
-  assert cfg.action_spec.num_values == ref.action_spec.num_values
+  assert tuple(cfg.timestep_spec.observation['WORLD.RGB'].shape) == tuple(ref.world_rgb_shape)
+  assert tuple(cfg.timestep_spec.observation['RGB'].shape) == tuple(ref.rgb_shape)
+  assert cfg.action_spec.num_values == ref.num_actions
 
 
 def test_territory_open_is_bounded_and_pays_for_claims(oracle):
@@ -89,29 +88,25 @@ def test_commons_closed_walls_keep_the_orchard_closed(oracle):
   assert eaten > 5
 
 
-@pytest.mark.skipif(compiler.reference_root() is None, reason='needs the reference checkout')
 def test_choice_prefabs_are_left_to_the_engine_unless_a_build_seed_fixes_them():
   # prefab_utils.lua:63-65: 'choice' is drawn with the env's random stream at every env build. Without a build seed the
   # blob carries the options (conditional objects) and the engine draws per env and episode; with one, a single draw is
   # baked into the blob (the older behaviour, still available for reproducing one fixed layout).
   from meltingpot_b200 import blob as blob_lib, substrates
-  per_env = compiler.compile_substrate('territory__inside_out', ('default',) * 5)
+  per_env = reference_configs.compile_recorded('territory__inside_out')
   sec = blob_lib.unpack(per_env)
   assert 'choice_groups' in sec and 'tr_res_cond' in sec and (sec['obj_choice'][:, 0] >= 0).sum() > 100
   assert per_env == substrates.load_blob('territory__inside_out', ('default',) * 5)  # the committed blob is this one
-  a = compiler.compile_substrate('territory__inside_out', ('default',) * 5, build_seed=1)
-  b = compiler.compile_substrate('territory__inside_out', ('default',) * 5, build_seed=2)
+  a = reference_configs.compile_recorded('territory__inside_out', build_seed=1)
+  b = reference_configs.compile_recorded('territory__inside_out', build_seed=2)
   assert a != b and 'choice_groups' not in blob_lib.unpack(a)
-  assert a == compiler.compile_substrate('territory__inside_out', ('default',) * 5, build_seed=1)
+  assert a == reference_configs.compile_recorded('territory__inside_out', build_seed=1)
 
 
-@pytest.mark.skipif(compiler.reference_root() is None, reason='needs the reference checkout')
 def test_role_tile_is_inert_for_default_roles_and_refused_when_it_would_pay(oracle):
   # component_library.lua:1098-1136: the tile pays rolesToRewards[role]; default builds carry role 'none'.
-  config = compiler.load_reference_config('commons_harvest__partnership')
-  settings = config.lab2d_settings_builder(roles=('default',) * 7, config=config)
-  import copy
-  paying = copy.deepcopy(compiler._plain(settings))
+  config = reference_configs.config('commons_harvest__partnership')
+  paying = reference_configs.settings('commons_harvest__partnership')
   for go in paying['simulation']['gameObjects']:
     for c in go['components']:
       if c['component'] == 'Role':

@@ -3,10 +3,10 @@
 import json
 
 import numpy as np
-import pytest
 
 from meltingpot_b200 import blob as mpb
-from meltingpot_b200 import compiler, substrates
+from meltingpot_b200 import substrates
+from tests import reference_configs
 
 
 def _tables(blob):
@@ -26,14 +26,14 @@ def test_layout_and_specs(coins_blob):
   assert list(dp[4:8]) == [1.0, 1.0, 0.0, -2.0]             # self match, self mismatch, other match, other mismatch
 
 
-@pytest.mark.skipif(compiler.reference_root() is None, reason='needs the reference checkout')
 def test_build_seed_fixes_the_python_side_randomness():
-  a = compiler.compile_substrate('coins', ('default',) * 2, build_seed=3)
-  assert a == compiler.compile_substrate('coins', ('default',) * 2, build_seed=3)
-  shapes = {tuple(int(v) for v in mpb.unpack(compiler.compile_substrate('coins', ('default',) * 2, build_seed=s))['co_ip'][:1])
+  # tests/golden records what coins' config builder returned after `random.seed(build_seed)` for build seeds 0-5
+  a = reference_configs.compile_recorded('coins', build_seed=3)
+  assert a == reference_configs.compile_recorded('coins', build_seed=3)
+  shapes = {tuple(int(v) for v in mpb.unpack(reference_configs.compile_recorded('coins', build_seed=s))['co_ip'][:1])
             for s in range(6)}
   assert len(shapes) > 1  # different seeds draw different map sizes (coin counts)
-  assert compiler.compile_substrate('coins', ('default',) * 2, build_seed=substrates.BUILD_SEEDS['coins']) == \
+  assert reference_configs.compile_recorded('coins', build_seed=substrates.BUILD_SEEDS['coins']) == \
       substrates.load_blob('coins', ('default',) * 2)
 
 

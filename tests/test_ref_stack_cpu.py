@@ -1,19 +1,17 @@
-"""The reference's own Python stack over this repo's `dmlab2d` boundary module (CPU: oracle backend; needs the checkout)."""
+"""This repo's `dmlab2d` boundary module against what the reference's own Python stack returned over it (CPU: oracle backend)."""
 
 import gzip
 import json
 import os
 import sys
-import unittest
 
 import numpy as np
 import pytest
 
 from meltingpot_b200 import compiler, lab2d_env
-from tests import ref_stack
+from tests import ref_stack, reference_configs
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-needs_reference = pytest.mark.skipif(compiler.reference_root() is None, reason='needs the reference checkout')
 
 
 def test_unflatten_inverts_flatten_and_str():
@@ -33,75 +31,58 @@ def test_unflatten_inverts_flatten_and_str():
   assert isinstance(back['simulation']['charPrefabMap'], dict)  # digit keys, still a dict
 
 
-@needs_reference
 @pytest.mark.parametrize('name,players', [('clean_up', 7), ('territory__rooms', 9), ('coins', 2)])
-def test_reference_stack_reproduces_the_committed_fixture(name, players):
+def test_oracle_backed_dmlab2d_module_reproduces_the_committed_fixture(name, players):
+  # tests/golden/ref_stack_<name>.json is what the reference's own stack returned over lab2d_env on the CPU oracle
+  # (tools/make_ref_stack_golden.py). Fed the flattened settings that stack's builder.py produced, the boundary module on
+  # the oracle must return the same raw observations, rewards and events, and the next episode's first step.
   with open(os.path.join(ROOT, 'tests', 'golden', f'ref_stack_{name}.json')) as f:
     want = json.load(f)
-  got = json.loads(json.dumps(ref_stack.run_reference_stack(name, players)))
-  got.pop('flat_settings')
-  assert got['class'] == 'meltingpot.utils.substrates.substrate.Substrate'  # the reference's class, not this repo's mirror
-  assert got == want
+  with gzip.open(os.path.join(ROOT, 'tests', 'golden', f'ref_stack_settings_{name}.json.gz')) as f:
+    flat = json.loads(f.read().decode())
+  lab = lab2d_env.Lab2d('', flat)
+  assert lab.env_seed == want['seed'] and lab.num_players == players
+
+  saved = lab2d_env.BACKEND_FACTORY
+  lab2d_env.BACKEND_FACTORY = ref_stack.OracleBackend
+  try:
+    with lab2d_env.Environment(env=lab, observation_names=lab.observation_names(), seed=lab.env_seed) as env:
+      ref_stack.check_raw_timestep(env.reset(), want['steps'][0], players, env)
+      for t, acts in enumerate(want['actions']):
+        action = {f'{i + 1}.{k}': np.int32(v) for i, a in enumerate(acts) for k, v in want['action_table'][a].items()}
+        ref_stack.check_raw_timestep(env.step(action), want['steps'][t + 1], players, env)
+    # the reference rebuilds the env with the next seed on every later reset (reset_wrapper.py:37-45, builder.py:174-187)
+    with lab2d_env.Environment(env=lab, observation_names=lab.observation_names(), seed=lab.env_seed + 1) as env:
+      ref_stack.check_raw_timestep(env.reset(), want['second_episode_first'], players, env)
+  finally:
+    lab2d_env.BACKEND_FACTORY = saved
 
 
-@needs_reference
 def test_compiling_from_flattened_settings_equals_compiling_from_the_config():
   # builder.py flattens the settings to "a.b.1.c" -> str for Lua (builder.py:55-67); lab2d_env un-flattens them. The blob
   # compiled from the round-tripped settings must equal the one compiled from the config's own settings.
-  config = compiler.load_reference_config('clean_up')
-  settings = compiler._plain(config.lab2d_settings_builder(roles=('default',) * 7, config=config))  # pylint: disable=protected-access
+  config = reference_configs.config('clean_up')
+  settings = reference_configs.settings('clean_up')
   flat = {k.replace('$', '.'): str(v) for k, v in lab2d_env.flatten_args(settings).items()}
   back = lab2d_env.unflatten_args(flat)
   assert compiler.compile_settings(back, config) == compiler.compile_settings(settings, config)
 
 
-@needs_reference
-@pytest.mark.parametrize('module', ['multiplayer_wrapper_test', 'discrete_action_wrapper_test', 'collective_reward_wrapper_test',
-                                    'collective_reward_wrapper_reset_test', 'observables_wrapper_test', 'reset_wrapper_test', 'base_test'])
-def test_reference_wrapper_unit_tests_pass_on_this_repos_dependency_shims(module):
-  # The reference's own wrapper tests (mocks of dmlab2d.Environment) run against this repo's dmlab2d / dm_env /
-  # immutabledict / reactivex stand-ins: the boundary module offers everything the wrappers touch.
-  import importlib
-  with ref_stack.reference_stack_on_oracle():
-    mod = importlib.import_module(f'meltingpot.utils.substrates.wrappers.{module}')
-    suite = unittest.defaultTestLoader.loadTestsFromModule(mod)
-    assert suite.countTestCases() > 0
-    result = unittest.TextTestRunner(stream=open(os.devnull, 'w'), verbosity=0).run(suite)
-    assert result.wasSuccessful(), [str(f[1])[-600:] for f in result.failures + result.errors][:2]
-
-
-@needs_reference
-def test_reference_import_leaves_no_stub_modules_behind():
-  compiler.load_reference_config('clean_up')
+def test_reference_import_leaves_no_stub_modules_behind(tmp_path):
+  # A stand-in checkout laid out like the reference: a config module that imports from meltingpot.utils.
+  pkg = tmp_path / 'meltingpot'
+  (pkg / 'configs' / 'substrates').mkdir(parents=True)
+  (pkg / 'utils' / 'substrates').mkdir(parents=True)
+  (pkg / 'utils' / 'substrates' / 'shapes.py').write_text("WALL = 'W'\n")
+  (pkg / 'configs' / 'substrates' / '__init__.py').write_text(
+      'import importlib\n\n\ndef get_config(name):\n'
+      "  return importlib.import_module(f'meltingpot.configs.substrates.{name}').get_config()\n")
+  (pkg / 'configs' / 'substrates' / 'clean_up.py').write_text(
+      'from meltingpot.utils.substrates import shapes\n\n\ndef get_config():\n  return shapes.WALL\n')
+  assert compiler.load_reference_config('clean_up', root=str(tmp_path)) == 'W'
   import meltingpot  # this repo's alias package, not a stub of the checkout
   assert 'meltingpot_b200' in (meltingpot.__doc__ or '') and hasattr(meltingpot, 'substrate')
   assert not [k for k in sys.modules if k.startswith('meltingpot.configs')]
-
-
-@needs_reference
-@pytest.mark.parametrize('name,players', ref_stack.SUBSTRATES)
-def test_reference_substrate_test_helper_accepts_the_stack(name, players):
-  # The reference's own conformance helper (meltingpot/testing/substrates.py:22-68, used by substrate_test.py:24-47 for
-  # every substrate): action / reward / discount / observation specs against an actual step, run on the reference's
-  # stack over this repo's dmlab2d module.
-  import importlib
-  with ref_stack.reference_stack_on_oracle():
-    helper = importlib.import_module('meltingpot.testing.substrates')
-    ref_substrate = importlib.import_module('meltingpot.substrate')
-    config = ref_substrate.get_config(name)
-    roles = (tuple(config.default_player_roles)[0],) * players
-    case = helper.SubstrateTestCase('assert_step_matches_specs')
-    env = ref_substrate.build(name, roles=roles)
-    try:
-      case.assert_step_matches_specs(env)
-      # substrate_test.py:41-47: the factory's per-player specs equal the env's
-      factory = ref_substrate.get_factory(name)
-      assert env.action_spec()[0] == factory.action_spec()
-      assert set(env.observation_spec()[0]) >= set(factory.timestep_spec().observation)
-      for key, spec in factory.timestep_spec().observation.items():
-        assert env.observation_spec()[0][key] == spec, key
-    finally:
-      env.close()
 
 
 @pytest.mark.parametrize('name,players', [('clean_up', 7), ('territory__rooms', 9)])
@@ -128,35 +109,30 @@ def test_boundary_module_compiles_builder_settings_and_refuses_to_run_without_a_
       lab2d_env.Environment(env=lab, observation_names=lab.observation_names(), seed=lab.env_seed)
 
 
-@needs_reference
 def test_flat_views_equal_the_reference_stacks_own_dmlab2d_stream():
-  # The reference's innermost ObservablesWrapper emits the raw action dicts and flat TimeSteps (observables_wrapper.py:43-58).
-  # meltingpot_b200.substrate.flat_action / flat_timestep (what this repo's Substrate emits on observables().dmlab2d) must
-  # rebuild exactly that stream from the multiplayer-level action and TimeStep.
-  import importlib
+  # tests/golden/dmlab2d_stream_clean_up.json: what the reference's innermost ObservablesWrapper emitted
+  # (observables_wrapper.py:43-58) while its stack played `actions` over lab2d_env on the CPU oracle. flat_action (what
+  # this repo's Substrate emits on observables().dmlab2d.action) must rebuild the action dicts its wrappers handed to
+  # dmlab2d; fed those dicts, the boundary module must return the recorded flat TimeSteps. (tests/test_gpu_ref_stack.py
+  # checks flat_timestep, through the Substrate's own stream, against the same recording.)
   from meltingpot_b200 import substrate as b200_substrate
-  with ref_stack.reference_stack_on_oracle():
-    ref_substrate = importlib.import_module('meltingpot.substrate')
-    config = ref_substrate.get_config('clean_up')
-    env = ref_substrate.build('clean_up', roles=('default',) * 7)
-    raw_ts, raw_act = [], []
-    env.observables().dmlab2d.timestep.subscribe(raw_ts.append)
-    env.observables().dmlab2d.action.subscribe(raw_act.append)
-    individual, global_names = list(config.individual_observation_names), list(config.global_observation_names)
-    action_set = [dict(a) for a in compiler._plain(config.action_set)]  # pylint: disable=protected-access
-    try:
-      rng = np.random.default_rng(2)
-      ts = env.reset()
-      for t in range(12):
-        mine = b200_substrate.flat_timestep(ts, individual, global_names)
-        ref = raw_ts[-1]
-        assert mine.step_type == ref.step_type and mine.reward == ref.reward and mine.discount == ref.discount
-        assert set(mine.observation) <= set(ref.observation)          # (the raw env offers every observation; the wrappers select)
-        for key, value in mine.observation.items():
-          assert np.array_equal(value, ref.observation[key]), key
-        acts = [int(a) for a in rng.integers(0, len(action_set), 7)]
-        ts = env.step(acts)
-        mine_act = b200_substrate.flat_action(acts, action_set)
-        assert set(mine_act) == set(raw_act[-1]) and all(int(mine_act[k]) == int(raw_act[-1][k]) for k in mine_act)
-    finally:
-      env.close()
+  with open(os.path.join(ROOT, 'tests', 'golden', 'dmlab2d_stream_clean_up.json')) as f:
+    want = json.load(f)
+  action_set = reference_configs.config('clean_up').action_set
+  for acts, rec in zip(want['actions'], want['raw_actions']):
+    mine = b200_substrate.flat_action(acts, action_set)
+    assert all(v.dtype == np.int32 and v.shape == () for v in mine.values())
+    assert {k: int(v) for k, v in mine.items()} == rec
+  with gzip.open(os.path.join(ROOT, 'tests', 'golden', 'ref_stack_settings_clean_up.json.gz')) as f:
+    lab = lab2d_env.Lab2d('', json.loads(f.read().decode()))
+  assert lab.env_seed == want['seed']
+  saved = lab2d_env.BACKEND_FACTORY
+  lab2d_env.BACKEND_FACTORY = ref_stack.OracleBackend
+  try:
+    with lab2d_env.Environment(env=lab, observation_names=lab.observation_names(), seed=lab.env_seed) as env:
+      got = [ref_stack.describe_raw_timestep(env.reset())]
+      for rec in want['raw_actions']:
+        got.append(ref_stack.describe_raw_timestep(env.step({k: np.int32(v) for k, v in rec.items()})))
+  finally:
+    lab2d_env.BACKEND_FACTORY = saved
+  assert got == want['raw_timesteps']
